@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's engine (one process per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path on the host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # + the last timed step's latents as DIR/*.npy
 
 A "step" is one iteration of src/pipelines/pipeline_diffsensei.py:310-337 — UNetMangaModel.forward at UNet batch
 B = 2*bs under CFG, the CFG blend and the DDIM update — for BASELINE.json configs[1]: 1024x1024 panels, bs = 4 per
@@ -43,6 +44,7 @@ METRIC = "unet_denoise_steps_per_sec_1024sq_bs4"
 UNIT = "steps/s"
 T_STEPS = 50
 GUIDANCE, IP_SCALE = 7.5, 0.6
+UNET_WEIGHT_SEED = 1234
 STEP_TFLOP_CFG2 = 54.8          # analytic 2*MAC count of one cfg2 step, SURVEY.md §8d / BASELINE.md §2
 
 
@@ -156,6 +158,18 @@ def synthetic_inputs(cfg, bs, h, w, n_chars, device, dialogs=False, mllm=False):
         d = DIALOG_BOXES + [[0.0] * 4] * 5
         dialog = torch.tensor([[[0.0] * 4] * 8] * bs + [d] * bs)
     return lat, ehs, pooled, time_ids, bbox, dialog
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of ``arrays`` (name -> tensor) as ``out_dir/<name>.npy`` in float32, so that two builds run
+    with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
 
 
 def event_time_ms(fn, iters, stream_sync=True):
@@ -620,10 +634,15 @@ def run_ours(args):
     peaks = measured_peaks()
     cfg = ds.SDXL_MANGA if args.config != "tiny" else ds.TINY
     groups = config_panels(args.config)
+    if args.dump_outputs:
+        # the dump's size follows from the shapes alone: every rank refuses the same run before any work is timed
+        dump_bytes = sum(bs * world * 4 * h * w * 4 for bs, h, w, *_ in groups)
+        if dump_bytes > DUMP_LIMIT_BYTES:
+            raise SystemExit(f"bench.py: --dump-outputs would write {dump_bytes} bytes, more than {DUMP_LIMIT_BYTES}")
 
     t0 = time.time()
     engine = ds.UNetMangaEngine(cfg, dev)
-    sd = random_state_dict(unet_param_shapes(cfg), seed=1234, device=dev, dtype=torch.bfloat16)
+    sd = random_state_dict(unet_param_shapes(cfg), seed=UNET_WEIGHT_SEED, device=dev, dtype=torch.bfloat16)
     engine.load_state_dict(sd)
     del sd
     torch.cuda.empty_cache()
@@ -665,6 +684,12 @@ def run_ours(args):
     ms = parallel.max_over_ranks(ms, dev)
     steps_per_sec = world * 1e3 / ms
     clocks = clk.summary()
+    if args.dump_outputs:
+        # the latents the last timed step left, taken before the legs below overwrite them
+        dump = {f"latents_{g[1] * 8}x{g[2] * 8}": parallel.gather_latents(st.latents_nchw(), [g[0]] * world)
+                for g, st in zip(groups, steppers)}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dump)
 
     # ---- e2e: the same call with HOST buffers (pinned), H2D + step + D2H inside the timed region
     hosts = [(torch.randn(g[0], 4, g[1], g[2]).pin_memory(), torch.empty(g[0], 4, g[1], g[2]).pin_memory())
@@ -881,7 +906,11 @@ def main():
                     help="concurrent kernel chains per GPU (default: DS_CHAINS env, else 2)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-kernel-rooflines", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the latents of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     return run_reference(args) if args.impl == "reference" else run_ours(args)

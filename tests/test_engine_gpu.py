@@ -201,27 +201,28 @@ def test_pipeline_call_surface(tiny):
 
 def test_resampler_matches_executed_reference():
     import diffsensei_b200 as ds
-    g = torch.load(os.path.join(GOLDEN, "resampler_tiny.pt"), weights_only=False)
+    from test_oracle_golden import resampler_case, sampled
+    g, sd, x, magi = resampler_case("resampler_tiny.pt")
     res = ds.ResamplerEngine(**g["kwargs"], device=DEV)
-    res.load_state_dict(g["state_dict"])
-    out = res(g["x"], g["magi"])
+    res.load_state_dict(sd)
+    out = res(x, magi)
     assert out.shape == (1, 80, 128) and res.dtype() == bf16
-    assert rel_l2(out.float(), g["out"]) < 2e-2
-    assert rel_l2(res(torch.zeros_like(g["x"]), torch.zeros_like(g["magi"])).float(), g["out_zero"]) < 2e-2
+    assert rel_l2(sampled(out.float(), g), g["out"]) < 2e-2
+    assert rel_l2(sampled(res(torch.zeros_like(x), torch.zeros_like(magi)).float(), g), g["out_zero"]) < 2e-2
 
 
 def test_resampler_shipped_config_matches_executed_reference():
     """The Resampler at the SHIPPED size (dim 1280, depth 4, 20 heads, 4 x (257 + 1) image tokens, 84 M params) on the
     GPU vs the reference's own resampler.py executed on the same seeded weights (tests/golden/resampler_full.pt)."""
     import diffsensei_b200 as ds
-    from test_oracle_golden import resampler_full_case
-    g, sd, x, magi = resampler_full_case()
+    from test_oracle_golden import resampler_case, sampled
+    g, sd, x, magi = resampler_case("resampler_full.pt")
     res = ds.ResamplerEngine(**g["kwargs"], device=DEV)
     res.load_state_dict(sd)
     out = res(x, magi)
     assert out.shape == (1, 80, 2048)
-    e1 = rel_l2(out.float(), g["out"])
-    e0 = rel_l2(res(torch.zeros_like(x), torch.zeros_like(magi)).float(), g["out_zero"])
+    e1 = rel_l2(sampled(out.float(), g), g["out"])
+    e0 = rel_l2(sampled(res(torch.zeros_like(x), torch.zeros_like(magi)).float(), g), g["out_zero"])
     print(f"shipped-config Resampler vs executed reference: rel-L2 {e1:.3e} (zero inputs: {e0:.3e})")
     assert e1 < 2e-2 and e0 < 2e-2
 
@@ -233,19 +234,55 @@ def test_qwen_resampler_matches_executed_reference(name):
     width 160 and LayerNorms over 5120 features."""
     import diffsensei_b200 as ds
     from oracle.qwen_resampler import seeded_case
+    from test_oracle_golden import sampled
     g = torch.load(os.path.join(GOLDEN, "qwen_resampler.pt"), weights_only=False)[name]
     _m, sd, x = seeded_case(g["kwargs"], g["seed"])
     eng = ds.QwenResamplerEngine(**g["kwargs"], device=DEV)
     eng.load_state_dict(sd)
     out = eng(x)
-    err = rel_l2(out.float(), g["out"])
+    err = rel_l2(sampled(out.float(), g), g["out"])
     print(f"QwenResampler[{name}] vs executed reference: rel-L2 {err:.3e}")
-    assert out.shape == g["out"].shape and err < 1.5e-2
+    assert out.shape == (2, g["kwargs"]["grid_size"] ** 2, g["kwargs"]["embed_dim"]) and err < 1.5e-2
 
 
 def test_smoke_entry_point():
     import __graft_entry__
     __graft_entry__.smoke()
+
+
+def test_bench_dumps_the_latents_of_its_last_timed_step(tmp_path):
+    """bench.py --dump-outputs after W warm-up and K timed steps: the latents of W + K denoise steps of the
+    benchmark's seeded weights and inputs, recomputed here."""
+    import subprocess
+    import sys
+
+    import numpy as np
+
+    import bench
+    import diffsensei_b200 as ds
+    from conftest import ROOT
+    from diffsensei_b200.weights import random_state_dict, unet_param_shapes
+    warmup, steps = 3, 2
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "tiny", "--steps", str(steps),
+                        "--warmup", str(warmup), "--no-panels", "--no-library-baseline", "--no-cpu-baseline",
+                        "--no-kernel-rooflines", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    (bs, h, w, n_chars, dialogs, mllm), = bench.config_panels("tiny")
+    got = np.load(tmp_path / f"latents_{h * 8}x{w * 8}.npy")
+    assert got.dtype == np.float32 and got.shape == (bs, 4, h, w)
+    engine = ds.UNetMangaEngine(ds.TINY, DEV)
+    engine.load_state_dict(random_state_dict(unet_param_shapes(ds.TINY), seed=bench.UNET_WEIGHT_SEED, device=DEV,
+                                             dtype=bf16))
+    engine.set_ip_scale(bench.IP_SCALE)
+    inp = bench.synthetic_inputs(ds.TINY, bs, h, w, n_chars, DEV, dialogs=dialogs, mllm=mllm)
+    st = ds.DiffSenseiPipeline(engine).make_stepper(*inp[:5], h / w, inp[5], bench.T_STEPS, bench.GUIDANCE)
+    for i in range(warmup + steps):
+        st.step(i)
+    want = st.latents_nchw().cpu()
+    assert rel_l2(torch.from_numpy(got), want) < 1e-6
+    st.step(warmup + steps)
+    assert rel_l2(torch.from_numpy(got), st.latents_nchw().cpu()) > 1e-3     # one step more is told apart
 
 
 # ------------------------------------------------------------------------------------------ round-2 additions

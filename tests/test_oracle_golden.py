@@ -78,14 +78,36 @@ def test_dialog_embed_matches_reference_including_bf16_truncation():
     assert dialog_boxes_to_pixels(bf.float().unsqueeze(0) * 0 + torch.tensor([0, 0, 0.9, 0.5]), 19, 152)[0][2] == 136
 
 
+def sampled(t, g):
+    """The elements of ``t`` a fixture stores: the seeded sample ``g["idx"]`` of a large output, else ``t`` whole."""
+    return t.flatten()[g["idx"].long()] if "idx" in g else t
+
+
+def resampler_case(name):
+    """Regenerate the weights / inputs of tests/golden/<name> from its seeds (tools/make_golden.py)."""
+    from diffsensei_b200.config import ResamplerConfig
+    from diffsensei_b200.weights import random_state_dict, resampler_param_shapes
+    g = _load(name)
+    rc = ResamplerConfig(**g["kwargs"])
+    sd = random_state_dict(resampler_param_shapes(rc), seed=g["weight_seed"], device="cpu")
+    sd = {k: v.to(torch.bfloat16).float() for k, v in sd.items()}
+    gx = torch.Generator().manual_seed(g["input_seed"])
+    x = torch.randn(1, 4, g["n_tokens"], rc.embedding_dim, generator=gx).to(torch.bfloat16).float()
+    magi = torch.randn(1, 4, rc.magi_embedding_dim, generator=gx).to(torch.bfloat16).float()
+    x[0, g["n_real"]:] = 0
+    magi[0, g["n_real"]:] = 0
+    return g, sd, x, magi
+
+
 def test_resampler_matches_reference():
-    g = _load("resampler_tiny.pt")
+    g, sd, x, magi = resampler_case("resampler_tiny.pt")
     m = OracleResampler(**g["kwargs"]).eval()
-    m.load_state_dict(g["state_dict"])
+    m.load_state_dict(sd)
     with torch.no_grad():
-        assert rel_l2(m(g["x"], g["magi"]), g["out"]) < 1e-5
-        assert rel_l2(m(torch.zeros_like(g["x"]), torch.zeros_like(g["magi"])), g["out_zero"]) < 1e-5
-    assert g["out"].shape == (1, 80, 128)
+        out = m(x, magi)
+        assert rel_l2(sampled(out, g), g["out"]) < 1e-5
+        assert rel_l2(sampled(m(torch.zeros_like(x), torch.zeros_like(magi)), g), g["out_zero"]) < 1e-5
+    assert out.shape == (1, 80, 128)
 
 
 def test_resampler_shipped_config_param_count():
@@ -95,34 +117,20 @@ def test_resampler_shipped_config_param_count():
     assert n == 83_978_752                        # SURVEY §8c (v)
 
 
-def resampler_full_case():
-    """Regenerate the weights / inputs of tests/golden/resampler_full.pt from its seeds (tools/make_golden.py)."""
-    import dataclasses
-    from diffsensei_b200.config import RESAMPLER
-    from diffsensei_b200.weights import random_state_dict, resampler_param_shapes
-    g = _load("resampler_full.pt")
-    assert g["kwargs"] == dataclasses.asdict(RESAMPLER)
-    sd = random_state_dict(resampler_param_shapes(RESAMPLER), seed=g["weight_seed"], device="cpu")
-    sd = {k: v.to(torch.bfloat16).float() for k, v in sd.items()}
-    gx = torch.Generator().manual_seed(g["input_seed"])
-    x = torch.randn(1, 4, 257, 1280, generator=gx).to(torch.bfloat16).float()
-    magi = torch.randn(1, 4, 768, generator=gx).to(torch.bfloat16).float()
-    x[0, g["n_real"]:] = 0
-    magi[0, g["n_real"]:] = 0
-    return g, sd, x, magi
-
-
 def test_resampler_shipped_config_matches_executed_reference():
     """configs/model/diffsensei.yaml Resampler (dim 1280, depth 4, 20 heads, 257 CLIP tokens + 1 Magi token per
     character, 83,978,752 params): oracle restatement vs the reference's own resampler.py executed on the same
     seeded weights / inputs."""
-    g, sd, x, magi = resampler_full_case()
+    import dataclasses
+    from diffsensei_b200.config import RESAMPLER
+    g, sd, x, magi = resampler_case("resampler_full.pt")
+    assert g["kwargs"] == dataclasses.asdict(RESAMPLER)
     m = OracleResampler(**g["kwargs"]).eval()
     m.load_state_dict(sd)
     assert sum(p.numel() for p in m.parameters()) == 83_978_752
     with torch.no_grad():
-        assert rel_l2(m(x, magi), g["out"]) < 1e-5
-        assert rel_l2(m(torch.zeros_like(x), torch.zeros_like(magi)), g["out_zero"]) < 1e-5
+        assert rel_l2(sampled(m(x, magi), g), g["out"]) < 1e-5
+        assert rel_l2(sampled(m(torch.zeros_like(x), torch.zeros_like(magi)), g), g["out_zero"]) < 1e-5
 
 
 @pytest.mark.parametrize("name", ["tiny", "input", "output"])
@@ -132,4 +140,4 @@ def test_qwen_resampler_oracle_matches_executed_reference(name):
     from oracle.qwen_resampler import seeded_case
     g = _load("qwen_resampler.pt")[name]
     m, _sd, x = seeded_case(g["kwargs"], g["seed"])
-    assert rel_l2(m(x), g["out"]) < 1e-5
+    assert rel_l2(sampled(m(x), g), g["out"]) < 1e-5

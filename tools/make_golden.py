@@ -75,6 +75,20 @@ class StubAttn:
                 "to_out_b": self.to_out[0].bias.detach().clone()}
 
 
+SAMPLE = 4096
+
+
+def sampled(case, **outputs):
+    """``case`` plus the outputs: whole when small, else the elements at one fixed, seeded sample of SAMPLE flat
+    indices (``case["idx"]``, shared by all outputs of the case) so that every fixture stays well under 1 MB."""
+    numel = next(iter(outputs.values())).numel()
+    if numel > SAMPLE:
+        idx = torch.randperm(numel, generator=torch.Generator().manual_seed(7))[:SAMPLE].sort().values.to(torch.int32)
+        case["idx"] = idx
+        outputs = {k: v.flatten()[idx.long()].clone() for k, v in outputs.items()}
+    return {**case, **outputs}
+
+
 @torch.no_grad()
 def main():
     os.makedirs(OUT, exist_ok=True)
@@ -162,39 +176,31 @@ def main():
                       "out": enc(stub, sample, db)})
     torch.save(cases, f"{OUT}/dialog_embed.pt")
 
-    # ------------------------------------------------------------------ Resampler (tiny config)
-    torch.manual_seed(3)
-    kw = dict(dim=128, depth=2, dim_head=64, heads=2, num_queries=16, num_dummy_tokens=16, embedding_dim=64,
-              magi_embedding_dim=32, output_dim=128, ff_mult=4)
-    model = rs.Resampler(**kw).eval()
-    x = torch.randn(1, 4, 33, 64)
-    magi = torch.randn(1, 4, 32)
-    x[0, 2:] = 0
-    magi[0, 2:] = 0
-    torch.save({"kwargs": kw, "state_dict": model.state_dict(), "x": x, "magi": magi, "out": model(x, magi),
-                "out_zero": model(torch.zeros_like(x), torch.zeros_like(magi))}, f"{OUT}/resampler_tiny.pt")
-    # ------------------------------------------------------------------ Resampler at the SHIPPED config
-    # (configs/model/diffsensei.yaml + scripts/demo/gradio_wo_mllm.py:174-185: 83,978,752 params).  The weights
-    # (336 MB) and inputs are NOT stored: both sides regenerate them from the seeds below with
-    # diffsensei_b200.weights.random_state_dict / torch.Generator (same torch build on the GPU box); only the
-    # reference's outputs are committed.
+    # ------------------------------------------------------------------ Resampler (tiny and SHIPPED config)
+    # shipped = configs/model/diffsensei.yaml + scripts/demo/gradio_wo_mllm.py:174-185: 83,978,752 params.  The weights
+    # and inputs are NOT stored: both sides regenerate them from the seeds below with
+    # diffsensei_b200.weights.random_state_dict / torch.Generator (tests/test_oracle_golden.py::resampler_case); only
+    # the reference's outputs are committed, a seeded sample of them where they are large.
     sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    from diffsensei_b200.config import RESAMPLER
+    from diffsensei_b200.config import RESAMPLER, RESAMPLER_TINY
     from diffsensei_b200.weights import random_state_dict, resampler_param_shapes
     import dataclasses
-    kwf = dataclasses.asdict(RESAMPLER)
-    full = rs.Resampler(**kwf).eval()
-    print("Resampler(shipped config) params:", sum(p.numel() for p in full.parameters()))
-    sdf = random_state_dict(resampler_param_shapes(RESAMPLER), seed=42, device="cpu")
-    sdf = {k: v.to(torch.bfloat16).float() for k, v in sdf.items()}      # bf16-representable on both sides
-    full.load_state_dict(sdf)
-    gx = torch.Generator().manual_seed(43)
-    xf = torch.randn(1, 4, 257, 1280, generator=gx).to(torch.bfloat16).float()
-    mf = torch.randn(1, 4, 768, generator=gx).to(torch.bfloat16).float()
-    xf[0, 3:] = 0                                                        # 3 real characters, 1 padded (:131-132)
-    mf[0, 3:] = 0
-    torch.save({"kwargs": kwf, "weight_seed": 42, "input_seed": 43, "n_real": 3, "out": full(xf, mf),
-                "out_zero": full(torch.zeros_like(xf), torch.zeros_like(mf))}, f"{OUT}/resampler_full.pt")
+    for fname, rc, wseed, iseed, n_tokens, n_real in (("resampler_tiny.pt", RESAMPLER_TINY, 3, 4, 33, 2),
+                                                      ("resampler_full.pt", RESAMPLER, 42, 43, 257, 3)):
+        kwr = dataclasses.asdict(rc)
+        model = rs.Resampler(**kwr).eval()
+        print(f"Resampler({fname}) params:", sum(p.numel() for p in model.parameters()))
+        sdr = random_state_dict(resampler_param_shapes(rc), seed=wseed, device="cpu")
+        sdr = {k: v.to(torch.bfloat16).float() for k, v in sdr.items()}      # bf16-representable on both sides
+        model.load_state_dict(sdr)
+        gx = torch.Generator().manual_seed(iseed)
+        x = torch.randn(1, 4, n_tokens, rc.embedding_dim, generator=gx).to(torch.bfloat16).float()
+        magi = torch.randn(1, 4, rc.magi_embedding_dim, generator=gx).to(torch.bfloat16).float()
+        x[0, n_real:] = 0                                                    # real characters, the rest padded (:131-132)
+        magi[0, n_real:] = 0
+        case = {"kwargs": kwr, "weight_seed": wseed, "input_seed": iseed, "n_tokens": n_tokens, "n_real": n_real}
+        torch.save(sampled(case, out=model(x, magi), out_zero=model(torch.zeros_like(x), torch.zeros_like(magi))),
+                   f"{OUT}/{fname}")
     # ------------------------------------------------------------------ QwenResampler (MLLM adaptor, §8f-4)
     # configs/model/diffsensei.yaml agent.input_resampler / output_resampler + a small one; weights / inputs are
     # regenerated from seeds on both sides (tests/test_oracle_golden.py::qwen_case), only outputs are stored
@@ -219,7 +225,7 @@ def main():
                 sdq[k] = (torch.randn(v.shape, generator=gq) * v.shape[-1] ** -0.5).to(torch.bfloat16).float()
         m.load_state_dict(sdq)
         xq = torch.randn(2, kw["grid_size"] ** 2, kw["kv_dim"], generator=gq).to(torch.bfloat16).float()
-        qcases[name] = {"kwargs": kw, "seed": 50, "out": m(xq)}
+        qcases[name] = sampled({"kwargs": kw, "seed": 50}, out=m(xq))
     torch.save(qcases, f"{OUT}/qwen_resampler.pt")
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
